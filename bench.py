@@ -6,9 +6,9 @@ on synthetic 16384x4 clouds, batch 16 per GPU (BASELINE.json configs[1]).
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
     python bench.py --impl reference ...      # the CPU restatement of the same path on the host cores
 
-One JSON line on rank 0.  A "step" is one batch of 16 scenes per GPU.  Every timed region times EXACTLY K steps between
-a barrier + synchronize on both sides (CUDA events, max over ranks) and is REPEATED R >= 3 times so that at least
-~1 s is timed per leg; the line reports the median repeat (and min / max).
+One JSON line on rank 0.  A "step" is one batch of 16 scenes per GPU.  Every timed region times EXACTLY K = --steps steps
+between a barrier + synchronize on both sides (CUDA events, max over ranks), so the same arguments time the same steps on the
+same inputs.  --dump-outputs DIR writes what the timed path (`value`) returned for its last step as DIR/<name>.npy.
 
   value         device-resident throughput: K steps through pointrcnn_b200.pipeline.BatchPipeline with `--inflight`
                 independent batches in flight (one CUDA graph per slot); inputs rotate through a pool larger than L2.
@@ -37,6 +37,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True    # the tree may be read-only: nothing is written there
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -285,9 +286,10 @@ def main():
     ap.add_argument("--no-eval", action="store_true", help="skip the end-to-end two-stage evaluation leg (BASELINE configs[4])")
     ap.add_argument("--inflight", type=int, default=6, help="independent batches in flight (CUDA streams); 1 = sequential")
     ap.add_argument("--graphs", type=int, default=1, help="1: one CUDA graph per pipeline slot (default), 0: eager launches")
-    ap.add_argument("--min-seconds", type=float, default=1.0, help="each leg repeats its K-step region until this much is timed (>= 3 repeats)")
     ap.add_argument("--pool", type=int, default=40, help="distinct input batches rotated through (40 x 4.2 MB > 126 MB L2)")
     ap.add_argument("--profile-out", default=None, help="write the line as indented JSON here as well")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the backbone features the timed path returned for its last step to DIR/*.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference_arm(args)
@@ -326,22 +328,15 @@ def main():
         if world > 1:
             dist.barrier()
 
-    def timed(run_k, min_seconds):
-        """repeat the K-step region (barrier + sync on both sides, CUDA events, max over ranks) until min_seconds are
-        timed, at least 3 times; returns the list of ms per step"""
+    def timed(run_k):
+        """time the K-step region once (barrier + sync on both sides, CUDA events, max over ranks); returns [ms per step]"""
         t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        out, total, offset = [], 0.0, 0
-        while len(out) < 3 or (total < min_seconds and len(out) < 200):
-            barrier(); torch.cuda.synchronize()
-            t0.record()
-            run_k(offset)
-            t1.record()
-            torch.cuda.synchronize(); barrier()
-            ms = max_over_ranks(t0.elapsed_time(t1), device=dev)      # identical on every rank -> same repeat count
-            out.append(ms / K)
-            total += ms * 1e-3
-            offset += K
-        return out
+        barrier(); torch.cuda.synchronize()
+        t0.record()
+        run_k(0)
+        t1.record()
+        torch.cuda.synchronize(); barrier()
+        return [max_over_ranks(t0.elapsed_time(t1), device=dev) / K]
 
     def summary(ms_list):
         return {"n": len(ms_list), "ms_per_step_median": statistics.median(ms_list), "ms_per_step_min": min(ms_list),
@@ -353,6 +348,15 @@ def main():
         rois, scores = res
         checksum[0] += float(scores.numpy().sum())       # the host consumer: touches every batch's proposals
         return None
+
+    def last_step_outputs():
+        """the (B,128,16384) features the timed path returned for its last step (with graphs: the replay's static output
+        of that step's slot), input batch (K-1) % P: all 16 scenes and channels at a fixed, seeded sample of 4096 points
+        (32 MB), plus the scene-mean feature of every channel over all points"""
+        feats = pipe.slots[(K - 1) % F].static_out[0] if G else pipe.run([dev_pool[(K - 1) % P]])[0]
+        cols = torch.from_numpy(np.sort(np.random.default_rng(0).choice(POINTS, 4096, replace=False))).to(dev)
+        return {"features_sample": feats.index_select(2, cols).float().cpu().numpy(),
+                "features_mean": feats.double().mean(2).cpu().numpy()}
 
     sampler = ClockSampler(local) if rank == 0 else None
     with torch.no_grad():
@@ -374,18 +378,18 @@ def main():
             sampler.mark()
 
         # ---------------- device-resident throughput: K steps, F independent batches in flight
-        ms_list = timed(lambda off: pipe.run([dev_pool[(off + i) % P] for i in range(K)], keep=False), args.min_seconds)
+        ms_list = timed(lambda off: pipe.run([dev_pool[(off + i) % P] for i in range(K)], keep=False))
         ms = statistics.median(ms_list)
+        dumped = last_step_outputs() if args.dump_outputs and rank == 0 else None
 
         # ---------------- end to end: pinned host input -> H2D -> backbone -> heads -> proposals -> D2H -> host consumer
-        e2e_list = timed(lambda off: pipe_rpn.run([host_pool[(off + i) % P] for i in range(K)], to_host=True, consume=consume_rois),
-                         args.min_seconds)
+        e2e_list = timed(lambda off: pipe_rpn.run([host_pool[(off + i) % P] for i in range(K)], to_host=True, consume=consume_rois))
         ms_e2e = statistics.median(e2e_list)
         d2h_bytes = BATCH * 100 * 7 * 4 + BATCH * 100 * 4
 
         # ---------------- secondary: the full feature tensor back on the host (PCIe bound)
         feat_list = timed(lambda off: pipe_feat.run([host_pool[(off + i) % P] for i in range(K)], to_host=True,
-                                                    consume=lambda i, r: None), 0.0)
+                                                    consume=lambda i, r: None))
         ms_feat = statistics.median(feat_list)
 
         # ---------------- strong scaling: global batch 16 -> 16/world scenes per GPU per step
@@ -396,7 +400,7 @@ def main():
             pipe_s = BatchPipeline(lambda x: net(x)[1], inflight=Fs, device=dev, graphs=G)
             small = [d[:bs] for d in dev_pool]
             pipe_s.run([small[i % P] for i in range(2 * Fs)], keep=False)
-            s_list = timed(lambda off: pipe_s.run([small[(off + i) % P] for i in range(K)], keep=False), args.min_seconds)
+            s_list = timed(lambda off: pipe_s.run([small[(off + i) % P] for i in range(K)], keep=False))
             ms_s = statistics.median(s_list)
             strong = {"global_batch": BATCH, "scenes_per_gpu_per_step": bs, "batches_in_flight": Fs, "ms_per_step": ms_s,
                       "value": BATCH / (ms_s * 1e-3), "unit": "scenes/s", "repeats": summary(s_list),
@@ -404,7 +408,7 @@ def main():
 
         # ---------------- sequential pass (one batch at a time, L2 flushed in between): per-batch latency and the
         # per-kernel-family breakdown (CUDA events on the launching stream)
-        KS = min(K, 10)
+        KS = K
         import gc
         gc.collect()                      # pinned buffers / graphs of the pipelined legs are released here, not inside a timed step
         for i in range(2):
@@ -454,7 +458,7 @@ def main():
         from pointrcnn_b200.train.step import RPNTrainer, synthetic_labels
         tr = RPNTrainer(input_channels=CHANNELS - 3, device=dev, world=world)
         labels = [synthetic_labels(dev_pool[i], seed=rank * 100 + i) for i in range(4)]
-        KT = min(K, 10)
+        KT = K
         for i in range(2):
             tr.step(dev_pool[i % 4], *labels[i % 4], grad_norm_clip=1.0)
         t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -514,7 +518,7 @@ def main():
         sys.path.insert(0, os.path.join(ROOT, "scripts"))
         try:
             import bench_rcnn_stage
-            rcnn = bench_rcnn_stage.measure(dev, steps=min(K, 10), warm=5)
+            rcnn = bench_rcnn_stage.measure(dev, steps=K, warm=5)
         except Exception as e:
             rcnn = {"unavailable": "%s: %s" % (type(e).__name__, e)}
         torch.cuda.empty_cache()
@@ -524,7 +528,7 @@ def main():
         sys.path.insert(0, os.path.join(ROOT, "scripts"))
         try:
             import bench_eval_e2e
-            eval_e2e = bench_eval_e2e.measure(dev, rank=rank, world=world, steps=min(K, 10), warm=3, barrier=barrier,
+            eval_e2e = bench_eval_e2e.measure(dev, rank=rank, world=world, steps=K, warm=3, barrier=barrier,
                                               max_over_ranks=max_over_ranks)
         except Exception as e:
             if world > 1:
@@ -546,7 +550,7 @@ def main():
                     for i in range(3):
                         ref_backbone(net, dev_pool[i % P])
                     torch.cuda.synchronize()
-                    KR = 5
+                    KR = K
                     evr = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(KR)]
                     for i, (a, b_) in enumerate(evr):
                         flush.fill_(1.0)
@@ -558,7 +562,7 @@ def main():
                     pipe_ref = BatchPipeline(lambda x: ref_backbone(net, x)[1], inflight=F, device=dev, graphs=False)
                     pipe_ref.run([dev_pool[i % P] for i in range(F)], keep=False)
                     torch.cuda.synchronize()
-                    KP = 2 * F
+                    KP = K
                     a, b_ = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                     a.record()
                     pipe_ref.run([dev_pool[i % P] for i in range(KP)], keep=False)
@@ -668,6 +672,10 @@ def main():
             "ref_cuda": ref_cuda, "vs_ref_cuda": vs_ref, "strong_scaling": strong, "train_step": train, "rcnn_stage": rcnn, "eval_e2e": eval_e2e}
     if args.profile_out:
         json.dump(line, open(args.profile_out, "w"), indent=1)
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(line))
 
 

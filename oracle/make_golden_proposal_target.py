@@ -4,8 +4,10 @@ Runs the reference's OWN lib/rpn/proposal_target_layer.py (imported unchanged fr
 with its two GPU extension entry points served by the CPU oracle (boxes_iou3d_gpu -> oracle.boxes_iou3d, roipool3d_gpu ->
 oracle.roipool3d), in the deterministic configuration (ROI_FG_AUG_TIMES = 0, AUG_DATA = False: the random jitter loop draws
 from the CUDA generator in the reference and cannot be reproduced off-device), and writes
-tests/golden/proposal_target_layer.npz.  TEST INFRASTRUCTURE ONLY.   python oracle/make_golden_proposal_target.py
+tests/golden/proposal_target_layer.npz (pooled rows stored as the indices of the input points they copy: see compact()).
+TEST INFRASTRUCTURE ONLY.   python oracle/make_golden_proposal_target.py
 """
+import hashlib
 import os
 import sys
 import types
@@ -44,6 +46,47 @@ def inputs(B=2, N=4096, M=512, C=8, n_gt=7, seed=300):
     seg = (rng.random((B, N)) > 0.5).astype(np.float32)
     depth = np.linalg.norm(xyz, axis=2).astype(np.float32)
     return dict(roi_boxes3d=rois, gt_boxes3d=gts, rpn_xyz=xyz, rpn_features=feat, seg_mask=seg, pts_depth=depth)
+
+
+def _sha(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def _pooled(idx, inp, rois):
+    """pts_feature and sampled_pts of the layer's output from the pooled point indices: each pooled row is an input point
+    (seg_mask, pts_depth / 70 - 0.5, rpn_features) and its coordinates relative to the RoI, rotated by -ry about y
+    (proposal_target_layer.py:48-54, kitti_utils.rotate_pc_along_y_torch), computed with the same torch CPU ops"""
+    R = idx.shape[0]
+    b = (np.arange(R) // (R // inp["rpn_xyz"].shape[0]))[:, None]
+    depth = (torch.from_numpy(inp["pts_depth"]) / 70.0 - 0.5).numpy()
+    feature = np.concatenate([inp["seg_mask"][b, idx][..., None], depth[b, idx][..., None], inp["rpn_features"][b, idx]], 2)
+    r = torch.from_numpy(rois)
+    pc = torch.from_numpy(inp["rpn_xyz"][b, idx]) - r[:, None, 0:3]
+    cosa, sina = torch.cos(r[:, 6]).view(-1, 1), torch.sin(r[:, 6]).view(-1, 1)
+    rot = torch.cat((torch.cat([cosa, -sina], 1).unsqueeze(1), torch.cat([sina, cosa], 1).unsqueeze(1)), 1)
+    pc[:, :, [0, 2]] = torch.matmul(pc[:, :, [0, 2]], rot.permute(0, 2, 1))
+    return feature, pc.numpy()
+
+
+def compact(res, inp):
+    """the stored form of the layer's output (the pooled arrays as int16 point indices + the SHA-256 of each)"""
+    R, S = res["pts_feature"].shape[:2]
+    B = inp["rpn_xyz"].shape[0]
+    rows = [{inp["rpn_features"][b][i].tobytes(): i for i in range(inp["rpn_features"].shape[1])} for b in range(B)]
+    idx = np.array([[rows[r // (R // B)][res["pts_feature"][r, s, 2:].tobytes()] for s in range(S)] for r in range(R)], np.int16)
+    out = {k: v for k, v in res.items() if k not in ("pts_feature", "sampled_pts")}
+    out.update(pooled_index=idx, pts_feature_sha256=np.array(_sha(res["pts_feature"])), sampled_pts_sha256=np.array(_sha(res["sampled_pts"])))
+    assert all(np.array_equal(expand(out, inp)[k], res[k]) for k in res)
+    return out
+
+
+def expand(g, inp):
+    """the layer's output from its stored form, checked bit for bit against the stored SHA-256"""
+    out = {k: g[k] for k in ("cls_label", "reg_valid_mask", "gt_of_rois", "gt_iou", "roi_boxes3d")}
+    out["pts_feature"], out["sampled_pts"] = _pooled(g["pooled_index"].astype(np.int64), inp, g["roi_boxes3d"])
+    for k in ("pts_feature", "sampled_pts"):
+        assert _sha(out[k]) == str(g[k + "_sha256"]), "%s does not rebuild from the stored indices" % k
+    return out
 
 
 def main():
@@ -86,7 +129,7 @@ def main():
     print("cls_label counts", {int(c): int((res["cls_label"] == c).sum()) for c in (-1, 0, 1)}, "reg_valid", int(res["reg_valid_mask"].sum()),
           "iou range", float(res["gt_iou"].min()), float(res["gt_iou"].max()))
     path = os.path.join(ROOT, "tests", "golden", "proposal_target_layer.npz")
-    np.savez_compressed(path, **res)
+    np.savez_compressed(path, **compact(res, inp))
     print("wrote", path, os.path.getsize(path))
 
 

@@ -271,6 +271,23 @@ print('OK')
     assert r.returncode == 0 and "OK" in r.stdout, r.stderr[-2000:]
 
 
+def test_network_layout_matches_the_reference():
+    """state_dict names, order and shapes of the RPN backbone and of the whole two-stage network equal those of the
+    reference's own Pointnet2MSG and PointRCNN (TEST mode, tools/cfgs/default.yaml), recorded from the reference's Python
+    by oracle/make_golden_layout.py: the reference's checkpoints load as they are"""
+    import json
+    from pointrcnn_b200.backbone import Pointnet2MSG
+    from pointrcnn_b200.point_rcnn import PointRCNNInference
+    gold = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_layout.json")))
+
+    def layout(net):
+        return [[k, list(v.shape)] for k, v in net.state_dict().items()]
+    assert layout(Pointnet2MSG(input_channels=0)) == gold["Pointnet2MSG(input_channels=0)"]
+    net = PointRCNNInference(input_channels=0)
+    assert layout(net) == gold["PointRCNN(num_classes=2, mode=TEST)"]
+    assert sum(p.numel() for p in net.parameters()) == gold["PointRCNN parameters"]
+
+
 def test_options_struct_matches_the_header():
     """ctypes mirror of struct prb_options: same fields, same order as include/pointrcnn_b200.h"""
     import re

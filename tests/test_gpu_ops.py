@@ -1,6 +1,7 @@
 """GPU parity tests (run with -m gpu on the B200 box): every native of the C ABI against
   (1) the CPU oracle (oracle/pointops_oracle.c, bit-exact for index work), and
-  (2) the reference's own CUDA kernels rebuilt for sm_100a (oracle/_ref) when that library is present.
+  (2) the reference's own CUDA kernels rebuilt for sm_100a (oracle/_ref): their recorded outputs (tests/refstore.py), and
+      the live kernels as well when that library is present.
 Calls go through the reference-named extension modules / Python wrappers, i.e. through the C ABI.
 """
 import os
@@ -9,6 +10,7 @@ import numpy as np
 import pytest
 import torch
 
+import refstore as REF
 import synth
 from oracle import oracle as O
 from oracle import refgpu as R
@@ -19,8 +21,6 @@ from pointrcnn_b200.ext import iou3d_cuda, roipool3d_cuda  # noqa: E402
 from pointrcnn_b200.iou3d import iou3d_utils  # noqa: E402
 from pointrcnn_b200.pointnet2 import pointnet2_utils as pu  # noqa: E402
 from pointrcnn_b200.roipool3d import roipool3d_utils  # noqa: E402
-
-HAVE_REF = R.available()
 
 
 def T(a, dev):
@@ -64,10 +64,8 @@ def test_fps_index_exact(cuda, B, N, M, kind):
     assert np.array_equal(idx2.cpu().numpy(), want)
     exp_xyz = np.stack([xyz[b][want[b]] for b in range(B)])
     assert np.array_equal(new_xyz.cpu().numpy(), exp_xyz), "emitted new_xyz != xyz[idx]"
-    if HAVE_REF:
-        ref, ref_temp = R.fps(x, M, return_temp=True)
-        assert torch.equal(got, ref), "FPS indices differ from the reference kernel"
-        assert np.array_equal(ref_temp.cpu().numpy(), want_temp), "oracle temp != reference temp"
+    REF.equal("idx", got, lambda: R.fps(x, M), "FPS indices differ from the reference kernel")
+    REF.equal("temp", want_temp, lambda: R.fps(x, M, return_temp=True)[1], "oracle temp != reference temp")
 
 
 @pytest.mark.parametrize("opt", [{"fps_cluster": 1}, {"fps_cluster": 2}, {"fps_cluster": 4}, {"fps_cluster": 8},
@@ -271,11 +269,13 @@ def test_fps_pruned_kernel_resumes_from_caller_temp(cuda, N, M, prune):
         pointnet2_cuda.furthest_point_sampling_wrapper(2, N, M, x, temp, idx)
     assert np.array_equal(idx.cpu().numpy(), want)
     assert np.array_equal(temp.cpu().numpy(), want_temp)
-    if HAVE_REF:
+    def ref_fps():
         rt = T(t0.copy(), cuda)
         ridx = torch.empty((2, M), dtype=torch.int32, device=cuda)
         R.fps_raw(x, rt, ridx)
-        assert torch.equal(ridx, idx) and torch.equal(rt, temp)
+        return ridx, rt
+    REF.equal("idx", idx, lambda: ref_fps()[0])
+    REF.equal("temp", temp, lambda: ref_fps()[1])
 
 
 # ------------------------------------------------------------------------------------------------ ball query / grouping
@@ -290,8 +290,7 @@ def test_ball_query_exact(cuda, kind, N, M, r, ns):
     x, c = T(xyz, cuda), T(new_xyz, cuda)
     got = pu.ball_query(r, ns, x, c)
     assert np.array_equal(got.cpu().numpy(), want)
-    if HAVE_REF:
-        assert torch.equal(got, R.ball_query(r, ns, x, c))
+    REF.equal("idx", got, lambda: R.ball_query(r, ns, x, c))
 
 
 def test_ball_query_no_hit_rows_stay_zero_and_msg2(cuda):
@@ -327,8 +326,7 @@ def test_group_gather_and_grads(cuda):
     go2 = rng.standard_normal((B, C, M)).astype(np.float32)
     pu.gather_operation(fr2, T(gidx, cuda)).backward(T(go2, cuda))
     np.testing.assert_allclose(fr2.grad.cpu().numpy(), O.gather_grad(go2, gidx, N), rtol=1e-5, atol=1e-5)
-    if HAVE_REF:
-        assert torch.equal(got, R.group(f, i))
+    REF.equal("group", got, lambda: R.group(f, i))
 
 
 # ------------------------------------------------------------------------------------------------ three_nn / interpolate
@@ -345,9 +343,8 @@ def test_three_nn_exact(cuda, n, m, kind):
     np.testing.assert_allclose(dist.cpu().numpy(), np.sqrt(d2), rtol=1e-6)
     if m >= 3:
         np.testing.assert_allclose(w.cpu().numpy(), O.interp_weights(d2), rtol=2e-6, atol=1e-7)
-    if HAVE_REF:
-        rd2, ridx = R.three_nn(u, k)
-        assert torch.equal(gi, ridx) and torch.equal(got_d2, rd2)
+    REF.equal("idx", gi, lambda: R.three_nn(u, k)[1])
+    REF.equal("dist2", got_d2, lambda: R.three_nn(u, k)[0])
 
 
 def test_three_interpolate_and_grad(cuda):
@@ -366,8 +363,7 @@ def test_three_interpolate_and_grad(cuda):
     go = rng.standard_normal((B, C, N)).astype(np.float32)
     pu.three_interpolate(fr, i, ww).backward(T(go, cuda))
     np.testing.assert_allclose(fr.grad.cpu().numpy(), O.three_interpolate_grad(go, idx, w, M), rtol=1e-4, atol=1e-4)
-    if HAVE_REF:
-        assert torch.equal(got, R.three_interpolate(f, i, ww))
+    REF.equal("out", got, lambda: R.three_interpolate(f, i, ww))
 
 
 # ------------------------------------------------------------------------------------------------ roipool3d
@@ -400,10 +396,9 @@ def test_roipool3d_vs_reference_and_oracle(cuda, B, N, M, C, S):
         with _cabi.options(**alt):
             roipool3d_cuda.forward(x, bx, f, p2, e2)
         assert torch.equal(p2, pooled) and torch.equal(e2, empty), "pass-B variant %r differs" % alt
-    if HAVE_REF and C > 0:
-        rp, re = R.roipool3d(x, f, bx, S)
-        assert torch.equal(empty, re), "empty flags differ from the reference kernel"
-        assert torch.equal(pooled, rp), "pooled rows differ from the reference kernel"
+    if C > 0:
+        REF.equal("empty", empty, lambda: R.roipool3d(x, f, bx, S)[1], "empty flags differ from the reference kernel")
+        REF.equal("pooled", pooled, lambda: R.roipool3d(x, f, bx, S)[0], "pooled rows differ from the reference kernel")
     # CPU oracle uses host libm for cos/sin: flags may differ only for points within 1e-4 m of a box face
     op, oe = O.roipool3d(xyz, feat, boxes, S)
     gp, ge = pooled.cpu().numpy(), empty.cpu().numpy()
@@ -494,9 +489,8 @@ def test_overlap_and_iou_matrices(cuda):
     np.testing.assert_allclose(ov.cpu().numpy(), want_ov, rtol=2e-4, atol=2e-4)
     np.testing.assert_allclose(iou.cpu().numpy(), want_iou, rtol=2e-4, atol=2e-5)
     assert (want_iou > 0.5).sum() > 50
-    if HAVE_REF:
-        assert torch.equal(ov, R.boxes_overlap_bev(ta, tb)), "overlap matrix not bit-identical to the reference kernel"
-        assert torch.equal(iou, R.boxes_iou_bev(ta, tb)), "IoU matrix not bit-identical to the reference kernel"
+    REF.equal("overlap", ov, lambda: R.boxes_overlap_bev(ta, tb), "overlap matrix not bit-identical to the reference kernel")
+    REF.equal("iou", iou, lambda: R.boxes_iou_bev(ta, tb), "IoU matrix not bit-identical to the reference kernel")
 
 
 @pytest.mark.parametrize("n,thresh,normal", [(100, 0.1, False), (1000, 0.3, False), (2700, 0.8, True), (6300, 0.8, True),
@@ -508,19 +502,17 @@ def test_nms_keep_exact(cuda, n, thresh, normal):
     keep = torch.zeros(n, dtype=torch.int64)
     num = (iou3d_cuda.nms_normal_gpu if normal else iou3d_cuda.nms_gpu)(tb, keep, thresh)
     got = keep[:num].numpy()
-    if HAVE_REF:
-        want = R.nms(tb, thresh, normal).numpy()
-        assert np.array_equal(got, want), "keep list differs from the reference nms"
-        rm = R.nms_mask(tb, thresh, normal).cpu().numpy().view(np.uint64)
-        from pointrcnn_b200 import _cabi as C
-        mask = torch.zeros((n, (n + 63) // 64), dtype=torch.int64, device=cuda)
-        C.check(C.lib().prb_nms_mask(C.ptr(tb), n, C.c_float(thresh), int(normal), C.ptr(mask), C.stream()), "nms_mask")
-        mm = mask.cpu().numpy().view(np.uint64)
-        rows = np.arange(n)[:, None] // 64
-        cols = np.arange(mm.shape[1])[None, :]
-        upper = cols >= rows
-        assert np.array_equal(mm[upper], rm[upper]), "upper-triangle mask differs from the reference kernel"
-        assert not mm[~upper].any()
+    REF.equal("keep", got, lambda: R.nms(tb, thresh, normal), "keep list differs from the reference nms")
+    from pointrcnn_b200 import _cabi as C
+    mask = torch.zeros((n, (n + 63) // 64), dtype=torch.int64, device=cuda)
+    C.check(C.lib().prb_nms_mask(C.ptr(tb), n, C.c_float(thresh), int(normal), C.ptr(mask), C.stream()), "nms_mask")
+    mm = mask.cpu().numpy().view(np.uint64)
+    rows = np.arange(n)[:, None] // 64
+    cols = np.arange(mm.shape[1])[None, :]
+    upper = cols >= rows
+    REF.equal("mask", mm[upper], lambda: R.nms_mask(tb, thresh, normal).cpu().numpy().view(np.uint64)[upper],
+              "upper-triangle mask differs from the reference kernel")
+    assert not mm[~upper].any()
     if normal:  # no transcendental in the axis-aligned IoU -> the CPU oracle is bit-exact too
         assert np.array_equal(got, O.nms(boxes, thresh, normal=True))
     else:
@@ -621,8 +613,7 @@ def test_fused_iou3d_matches_the_reference_sequence(cuda, M, N):
     got = iou3d_cuda.boxes_iou3d(a, b)
     mirror = iou3d_utils.boxes_iou3d_gpu(a, b)                          # the op-by-op mirror on this repo's overlap kernel
     assert torch.equal(got, mirror), "fused IoU differs from the op-by-op sequence"
-    if HAVE_REF:
-        assert torch.equal(got, _ref_iou3d(a, b)), "fused IoU differs from the reference sequence on the reference kernel"
+    REF.equal("iou3d", got, lambda: _ref_iou3d(a, b), "fused IoU differs from the reference sequence on the reference kernel")
     want = O.boxes_iou3d(b3[:M], b3[M:])
     np.testing.assert_allclose(got.cpu().numpy(), want, rtol=2e-4, atol=2e-6)      # CPU libm vs device sin/cos/atan2
     # batched form = per-scene calls; aligned form = the diagonal of the matrix
