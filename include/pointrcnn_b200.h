@@ -207,6 +207,14 @@ PRB_API int prb_sa_group_mlp_max_ws(int b, int n, int npoint, int nsample, int c
                                     const float *new_xyz, const float *feats_pm, const int *idx,
                                     const prb_mlp_desc *mlp, float *out, float *out_pm, int out_stride_c,
                                     int out_c_off, void *workspace, size_t workspace_bytes, void *stream);
+/* SA chains with c_feat <= 5: layer 0 is evaluated by the gather warps (CUDA cores) and only layers 1 .. L-1 run on the
+ * tensor core.  l0_w: (c0, 8) device floats per layer-0 channel [wx, wy, wz, wf0 .. wf4] (BN scale folded in, zero beyond
+ * 3 + c_feat), l0_shift: c0 device floats; `mlp`: layers 1 .. L-1 packed as plain rows (kind 2, c_in = c0), scale NULL.
+ * Same output as prb_sa_group_mlp_max_ws up to fp32 summation order; the chain must fit one launch (no workspace). */
+PRB_API int prb_sa_group_mlp_max_l0(int b, int n, int npoint, int nsample, int c_feat, const float *xyz,
+                                    const float *new_xyz, const float *feats_pm, const int *idx, int c0,
+                                    const float *l0_w, const float *l0_shift, const prb_mlp_desc *mlp, float *out,
+                                    float *out_pm, int out_stride_c, int out_c_off, void *stream);
 PRB_API int prb_fp_interp_mlp_ws(int b, int n, int m, int c_known, int c_skip, const float *known_pm,
                                  const int *idx, const float *weight, const float *skip,
                                  const prb_mlp_desc *mlp, float *out, float *out_pm, void *workspace,

@@ -16,6 +16,9 @@ constexpr int MAX_LAYERS = 3;
 constexpr int MAX_NP = 512;
 
 enum { IN_SA = 0, IN_FP = 1, IN_DIRECT = 2 };
+// kernel build of IN_SA whose gather warps evaluate layer 0 themselves (ChainParams.sa_l0); not a ChainParams.mode_in value
+enum { IN_SA_L0 = 3 };
+constexpr int L0_IN = 8;             // layer-0 inputs of the direct form: [dx, dy, dz, up to 5 feature channels]
 enum { OUT_ROWS = 0, OUT_SA_MAX = 1, OUT_FP = 2 };
 
 struct ChainParams {
@@ -48,6 +51,11 @@ struct ChainParams {
     int n, npoint, ns, log_ns, c_feat;
     const float *xyz, *new_xyz, *feats_pm;
     const int *idx;
+    // SA, layer 0 in the gather warps (c_feat <= 5): the gather warps write relu_tf32(W0 . [dxyz, f] + shift0) into the A
+    // ring, so the tensor-core chain starts at the original layer 1 (K = l0_np).  l0_w: l0_c rows of L0_IN floats (BN scale
+    // folded, not yet rounded), l0_shift: l0_c floats; padded to l0_np (multiple of KC) with zeros in shared memory
+    int sa_l0, l0_c, l0_np;
+    const float *l0_w, *l0_shift;
     // FP
     int m, c_known, c_skip;
     const float *known_pm, *weight, *skip;

@@ -47,9 +47,20 @@ struct PipeSmem {
 };
 
 // `pool`: the max-pool staging tiles exist only for SA outputs (the last region of the layout: other modes never touch it)
-__host__ __device__ inline size_t pipe_smem_bytes(int ne, int na, int nb0, int b0_bytes, int nb1, int b1_bytes, int np_total, bool pool) {
+// `l0_np`: layer-0 channels evaluated by the gather warps (ChainParams.sa_l0), L0_IN weights + 1 shift each; 0 otherwise
+__host__ __device__ inline size_t pipe_smem_bytes(int ne, int na, int nb0, int b0_bytes, int nb1, int b1_bytes, int np_total, bool pool,
+                                                  int l0_np) {
     return 1024 /*alignment slack*/ + (size_t)na * A_STAGE_BYTES + (size_t)nb0 * b0_bytes + (size_t)nb1 * b1_bytes +
-           (size_t)2 * np_total * sizeof(float) + (pool ? (size_t)ne * (TM * POOL_STRIDE + 8 * 16) * sizeof(float) : 0) + 64;
+           (size_t)l0_np * (L0_IN + 1) * sizeof(float) + (size_t)2 * np_total * sizeof(float) +
+           (pool ? (size_t)ne * (TM * POOL_STRIDE + 8 * 16) * sizeof(float) : 0) + 64;
+}
+
+// round to tf32, nearest with ties away from zero: the same bits as the host packer's tf32_rna_host (mlp_tc.cu), so that
+// layer-0 weights evaluated on the CUDA cores are the operands the tensor core would have seen
+__device__ __forceinline__ float tf32_rna_bits(float x) {
+    uint32_t u = __float_as_uint(x);
+    if ((u & 0x7f800000u) != 0x7f800000u) u += 0x1000u;
+    return __uint_as_float(u & 0xffffe000u);
 }
 
 __device__ __forceinline__ void bar_named(int id, int nthreads) {
@@ -278,7 +289,9 @@ __global__ void __launch_bounds__((NE + NGW + 1) * 128, MINB) mlp_pipe_kernel(co
     uint8_t *sA = base;
     uint8_t *sB0 = sA + (size_t)p.na * A_STAGE_BYTES;
     uint8_t *sB1 = sB0 + (size_t)p.nb0 * p.b0_stage_bytes;
-    float *s_scale = reinterpret_cast<float *>(sB1 + (size_t)p.nb1 * p.b1_stage_bytes);
+    float *s_l0w = reinterpret_cast<float *>(sB1 + (size_t)p.nb1 * p.b1_stage_bytes);   // IN_SA_L0: l0_np x L0_IN weights
+    float *s_l0sh = s_l0w + (size_t)p.l0_np * L0_IN;                                     // ... and l0_np shifts
+    float *s_scale = s_l0sh + p.l0_np;
     float *s_shift = s_scale + np_total;
     float *s_pool = s_shift + np_total;                                  // NE x (TM x POOL_STRIDE + 8 x 16)
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -300,6 +313,10 @@ __global__ void __launch_bounds__((NE + NGW + 1) * 128, MINB) mlp_pipe_kernel(co
     if (warp == W_MISC + 2) tmem_alloc(s2u(&S.tmem_base), (uint32_t)p.tmem_cols);
     for (int l = 0; l < L; ++l)
         for (int i = tid; i < p.np[l]; i += NTHREADS) { s_scale[sc_off(l) + i] = p.unit_scale ? 1.f : p.scale[l][i]; s_shift[sc_off(l) + i] = p.shift[l][i]; }
+    if (MIN == IN_SA_L0) {
+        for (int i = tid; i < p.l0_np * L0_IN; i += NTHREADS) s_l0w[i] = (i / L0_IN) < p.l0_c ? tf32_rna_bits(p.l0_w[i]) : 0.f;
+        for (int i = tid; i < p.l0_np; i += NTHREADS) s_l0sh[i] = i < p.l0_c ? p.l0_shift[i] : 0.f;
+    }
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -501,7 +518,7 @@ __global__ void __launch_bounds__((NE + NGW + 1) * 128, MINB) mlp_pipe_kernel(co
         RingPos ra = {0, 0};
         uint32_t cc = 0, it = 0;
         Cursor cur;
-        if (MIN == IN_SA) cur.init(tile0 * (TM >> p.log_ns), tstep * (TM >> p.log_ns), p.npoint);
+        if (MIN == IN_SA || MIN == IN_SA_L0) cur.init(tile0 * (TM >> p.log_ns), tstep * (TM >> p.log_ns), p.npoint);
         else if (MIN == IN_FP) cur.init(tile0 * TM, tstep * TM, p.n);
         else cur.init(0, 0, 1);
         for (int tile = tile0; tile < ntiles; tile += tstep, ++it, cur.advance()) {
@@ -512,7 +529,7 @@ __global__ void __launch_bounds__((NE + NGW + 1) * 128, MINB) mlp_pipe_kernel(co
             float cx = 0.f, cy = 0.f, cz = 0.f;
             int my_scene = 0, my_u = 0;
             const int par = it & 1;
-            if (MIN == IN_SA) {
+            if (MIN == IN_SA || MIN == IN_SA_L0) {
                 int sc, pp;
                 cur.at(r >> p.log_ns, sc, pp);
                 if (valid) {
@@ -538,6 +555,23 @@ __global__ void __launch_bounds__((NE + NGW + 1) * 128, MINB) mlp_pipe_kernel(co
                 }
                 // one barrier per item: the table is double buffered, so the readers of item it-1 never see item it+1's rows
                 bar_named(5, 128 * NGW);
+            }
+            // IN_SA_L0: my row's layer-0 inputs [dx, dy, dz, f0..f4], rounded to tf32 as the A operand of the MMA form is
+            float in0[L0_IN];
+            if (MIN == IN_SA_L0) {
+#pragma unroll
+                for (int k = 0; k < L0_IN; ++k) in0[k] = 0.f;
+                if (valid) {
+                    const float *q = p.xyz + (size_t)src * 3;
+                    in0[0] = to_tf32(__ldg(q + 0) - cx);
+                    in0[1] = to_tf32(__ldg(q + 1) - cy);
+                    in0[2] = to_tf32(__ldg(q + 2) - cz);
+                    const int cf = p.c_feat;
+                    const float *f = p.feats_pm + (size_t)src * cf;
+#pragma unroll
+                    for (int k = 0; k < L0_IN - 3; ++k)
+                        if (k < cf) in0[3 + k] = to_tf32(__ldg(f + k));
+                }
             }
             // sources of the 8 rows my lane group helps to gather (rows of my own warp: shuffles instead of a table)
             int s8[8];
@@ -637,6 +671,41 @@ __global__ void __launch_bounds__((NE + NGW + 1) * 128, MINB) mlp_pipe_kernel(co
                             *reinterpret_cast<float4 *>(A + swz(rr, j8)) = v;
                         }
                     }
+                } else if (MIN == IN_SA_L0) {
+                    // layer 0 on the CUDA cores, one row per lane: channels k0 .. k0+31 = relu_tf32(W0 . in0 + shift0), written
+                    // as the 128-byte A row of the first MMA layer (the original layer 1).  Weights and shifts are broadcast
+                    // shared-memory reads; padding channels have zero weights and shifts, padding rows are zero.
+                    tt.timed(0, [&] { bwait_lazy(empty_bar, empty_par, lazy); });
+                    const float4 *w4 = reinterpret_cast<const float4 *>(s_l0w + (size_t)k0 * L0_IN);
+                    const float4 *sh4 = reinterpret_cast<const float4 *>(s_l0sh + k0);
+                    auto chunk = [&](auto wide_c) {
+                        constexpr bool WIDE = decltype(wide_c)::value;      // more than one feature channel: 8 inputs, else 4
+#pragma unroll
+                        for (int j = 0; j < 8; ++j) {
+                            const float4 b = sh4[j];
+                            float o[4];
+#pragma unroll
+                            for (int q = 0; q < 4; ++q) {
+                                const float4 wa = w4[2 * (4 * j + q)];
+                                float acc = __fmul_rn(wa.x, in0[0]);
+                                acc = __fmaf_rn(wa.y, in0[1], acc);
+                                acc = __fmaf_rn(wa.z, in0[2], acc);
+                                acc = __fmaf_rn(wa.w, in0[3], acc);
+                                if (WIDE) {
+                                    const float4 wb = w4[2 * (4 * j + q) + 1];
+                                    acc = __fmaf_rn(wb.x, in0[4], acc);
+                                    acc = __fmaf_rn(wb.y, in0[5], acc);
+                                    acc = __fmaf_rn(wb.z, in0[6], acc);
+                                    acc = __fmaf_rn(wb.w, in0[7], acc);
+                                }
+                                const float t = q == 0 ? b.x : q == 1 ? b.y : q == 2 ? b.z : b.w;
+                                o[q] = valid ? relu_to_tf32(acc + t) : 0.f;
+                            }
+                            *reinterpret_cast<float4 *>(A + swz(r, j)) = make_float4(o[0], o[1], o[2], o[3]);
+                        }
+                    };
+                    if (p.c_feat > 1) chunk(std::true_type{});
+                    else chunk(std::false_type{});
                 } else if (MIN == IN_SA) {
                     // relative xyz segment: [x - cx, y - cy, z - cz, (<= 5 feature channels,) 0 ...]; one K=8 step
                     float4 v = make_float4(0.f, 0.f, 0.f, 0.f), v2 = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -1088,7 +1157,7 @@ static bool pipe_plan(const ChainParams &p, int max_optin, PipePlan *out, int fo
             if (o.mlp_occ == 1 || force_occ == 1) pl.occ = 1;
             if (force_occ == 2 && pl.occ != 2) continue;
             if (force_occ == 3) {                          // three CTAs per SM: <= 128 columns each, SA gather without row segments
-                if (cols > 128 || p.mode_in != IN_SA || p.mode_out != OUT_SA_MAX || p.c_feat > 5 || !(p.ns == 16 || p.ns == 32)) continue;
+                if (cols > 128 || p.mode_in != IN_SA || p.mode_out != OUT_SA_MAX || p.c_feat > 5 || !(p.ns == 16 || p.ns == 32)) continue;   // also the IN_SA_L0 build
                 pl.occ = 3;
             }
             pl.ne = pl.ngw = pl.occ >= 2 ? 1 : 2;         // builds: 4+4 row warps x 2 (or 3) CTAs, or 8+8 row warps x 1 CTA
@@ -1122,7 +1191,7 @@ static bool pipe_plan(const ChainParams &p, int max_optin, PipePlan *out, int fo
                     const int na_min = k0 + 1 < PIPE_MAX_A ? (k0 + 1 > 3 ? k0 + 1 : 3) : PIPE_MAX_A;
                     for (int na = (k0 + 2 < PIPE_MAX_A ? (k0 + 2 > 3 ? k0 + 2 : 3) : PIPE_MAX_A); na >= na_min && !ok; --na) {
                         const size_t smem = pipe_smem_bytes(pl.ne, na, st0, pl.b0_bytes, st1, pl.b1_bytes, np_total,
-                                                            p.mode_out == OUT_SA_MAX && !(p.ns == 16 || p.ns == 32));
+                                                            p.mode_out == OUT_SA_MAX && !(p.ns == 16 || p.ns == 32), p.sa_l0 ? p.l0_np : 0);
                         if (smem <= budget && smem <= (size_t)max_optin) {
                             pl.na = na; pl.nb0 = st0; pl.nb1 = st1; pl.smem = smem; pl.resident = 1; ok = true;
                         }
@@ -1133,7 +1202,8 @@ static bool pipe_plan(const ChainParams &p, int max_optin, PipePlan *out, int fo
             for (int nb = 3; nb >= 2 && !ok; --nb)
                 for (int na = (k0 + 2 < PIPE_MAX_A ? (k0 + 2 > 3 ? k0 + 2 : 3) : PIPE_MAX_A); na >= 2 && !ok; --na) {
                     const size_t smem = pipe_smem_bytes(pl.ne, na, nb, pl.b0_bytes, L > 1 ? nb : 0, pl.b1_bytes, np_total,
-                                                        p.mode_out == OUT_SA_MAX && !(p.ns == 16 || p.ns == 32));   // 16 / 32 samples pool in registers
+                                                        p.mode_out == OUT_SA_MAX && !(p.ns == 16 || p.ns == 32),   // 16 / 32 samples pool in registers
+                                                        p.sa_l0 ? p.l0_np : 0);
                     if (smem <= budget && smem <= (size_t)max_optin && (nb == 2 || na >= (k0 < 4 ? k0 : 4))) {
                         pl.na = na; pl.nb0 = nb; pl.nb1 = L > 1 ? nb : 0; pl.smem = smem; ok = true;
                     }
@@ -1180,10 +1250,11 @@ static int launch_with_plan(ChainParams &p, const PipePlan &pl, cudaStream_t st)
     } while (0)
 #define PRB_LAUNCH_PIPE_IO(NE, NGW, MB)                                                                    \
     do {                                                                                                   \
-        const int key = p.mode_in * 3 + p.mode_out;                                                        \
+        const int key = (p.sa_l0 ? IN_SA_L0 : p.mode_in) * 3 + p.mode_out;                                \
         switch (key) {                                                                                     \
             case IN_SA * 3 + OUT_ROWS: PRB_LAUNCH_PIPE(NE, NGW, MB, IN_SA, OUT_ROWS); break;              \
             case IN_SA * 3 + OUT_SA_MAX: PRB_LAUNCH_PIPE(NE, NGW, MB, IN_SA, OUT_SA_MAX); break;          \
+            case IN_SA_L0 * 3 + OUT_SA_MAX: PRB_LAUNCH_PIPE(NE, NGW, MB, IN_SA_L0, OUT_SA_MAX); break;    \
             case IN_FP * 3 + OUT_ROWS: PRB_LAUNCH_PIPE(NE, NGW, MB, IN_FP, OUT_ROWS); break;              \
             case IN_FP * 3 + OUT_FP: PRB_LAUNCH_PIPE(NE, NGW, MB, IN_FP, OUT_FP); break;                  \
             case IN_DIRECT * 3 + OUT_ROWS: PRB_LAUNCH_PIPE(NE, NGW, MB, IN_DIRECT, OUT_ROWS); break;      \
@@ -1192,7 +1263,8 @@ static int launch_with_plan(ChainParams &p, const PipePlan &pl, cudaStream_t st)
             default: set_error("mlp: unsupported input / output mode pair %d / %d", p.mode_in, p.mode_out); return -1; \
         }                                                                                                  \
     } while (0)
-    if (pl.occ == 3) PRB_LAUNCH_PIPE(1, 1, 3, IN_SA, OUT_SA_MAX);
+    if (pl.occ == 3 && p.sa_l0) PRB_LAUNCH_PIPE(1, 1, 3, IN_SA_L0, OUT_SA_MAX);
+    else if (pl.occ == 3) PRB_LAUNCH_PIPE(1, 1, 3, IN_SA, OUT_SA_MAX);
     else if (pl.ne == 1 && pl.ngw == 1) PRB_LAUNCH_PIPE_IO(1, 1, 2);      // launch bounds only cap the registers; occ 1 runs the same build
     else if (pl.ngw == 3) PRB_LAUNCH_PIPE_IO(2, 3, 1);
     else PRB_LAUNCH_PIPE_IO(2, 2, 1);
@@ -1245,7 +1317,7 @@ int launch_chain_pipe(ChainParams &p, cudaStream_t st) {
     if (nc > 1) {
         TuneKey key;
         memset(&key, 0, sizeof(key));
-        key.dev = dev; key.mode_in = p.mode_in; key.mode_out = p.mode_out; key.L = p.num_layers; key.ns = p.ns;
+        key.dev = dev; key.mode_in = p.sa_l0 ? IN_SA_L0 : p.mode_in; key.mode_out = p.mode_out; key.L = p.num_layers; key.ns = p.ns;
         key.k0 = p.nchunks[0]; key.tiles = p.num_tiles;
         for (int l = 0; l < p.num_layers; ++l) key.np[l] = p.np[l];
         int choice = 0;
@@ -1300,7 +1372,8 @@ int pipe_tuned_plans(int *dst, int max_entries) {
         if (n >= max_entries) break;
         const TuneKey &k = kv.first;
         int *d = dst + 18 * n++;
-        d[0] = k.mode_in; d[1] = k.mode_out; d[2] = k.L; d[3] = k.ns; d[4] = k.k0; d[5] = k.tiles; d[6] = k.np[0]; d[7] = k.np[1]; d[8] = k.np[2];
+        d[0] = k.mode_in == IN_SA_L0 ? IN_SA : k.mode_in;       // reported as an SA chain (one layer shorter)
+        d[1] = k.mode_out; d[2] = k.L; d[3] = k.ns; d[4] = k.k0; d[5] = k.tiles; d[6] = k.np[0]; d[7] = k.np[1]; d[8] = k.np[2];
         d[9] = kv.second.choice;
         for (int c = 0; c < 4; ++c) {       // candidates: build code (0 = none) and measured microseconds
             d[10 + 2 * c] = c < kv.second.nc ? kv.second.code[c] : 0;

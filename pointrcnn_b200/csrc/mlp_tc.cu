@@ -1001,6 +1001,42 @@ PRB_API int prb_sa_group_mlp_max_ws(int b, int n, int npoint, int nsample, int c
     return run_chain(io, mlp, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
+// SA chains with c_feat <= 5, layer 0 outside the tensor core: the gather warps evaluate relu(W0 . [x_j - c, f_j] + shift0)
+// (l0_w: c0 x 8 floats per channel [wx, wy, wz, wf0 .. wf4], BN scale folded, zero beyond 3 + c_feat; l0_shift: c0 floats;
+// both device) and write it as the A operand of `mlp`, the chain of the original layers 1 .. L-1 packed as plain rows
+// (kind 2, c_in = c0).  One tensor-memory hand-off per tile fewer than prb_sa_group_mlp_max_ws with the same operands
+// (tf32-rounded inputs and weights); the chain must fit one launch.
+PRB_API int prb_sa_group_mlp_max_l0(int b, int n, int npoint, int nsample, int c_feat, const float *xyz, const float *new_xyz,
+                                    const float *feats_pm, const int *idx, int c0, const float *l0_w, const float *l0_shift,
+                                    const prb_mlp_desc *mlp, float *out, float *out_pm, int out_stride_c, int out_c_off, void *stream) {
+    PRB_REQUIRE(b >= 0 && n > 0 && npoint > 0 && nsample > 0 && xyz && new_xyz && idx && mlp && out && l0_w && l0_shift,
+                "sa_group_mlp_max_l0: bad arguments");
+    PRB_REQUIRE(c_feat >= 0 && c_feat <= L0_IN - 3, "sa_group_mlp_max_l0: c_feat %d > %d", c_feat, L0_IN - 3);
+    PRB_REQUIRE(c_feat == 0 || feats_pm, "sa_group_mlp_max_l0: features missing");
+    PRB_REQUIRE(c0 >= 1 && c0 <= MAX_NP && mlp->c_in == c0, "sa_group_mlp_max_l0: layer-0 width %d / chain input %d", c0, mlp->c_in);
+    PRB_REQUIRE(mlp->scale == nullptr, "sa_group_mlp_max_l0: the BN scale must be folded into the weights");
+    PRB_REQUIRE(nsample >= 4 && nsample <= 128 && (nsample & (nsample - 1)) == 0, "sa_group_mlp_max_l0: nsample %d must be a power of two in [4,128]", nsample);
+    PRB_REQUIRE(use_pipe(), "sa_group_mlp_max_l0: needs the pipelined kernel (mlp_pipeline = 1, mlp_gather = 0)");
+    const int L = mlp->num_layers;
+    PRB_REQUIRE(L >= 1 && L <= MAX_LAYERS, "sa_group_mlp_max_l0: num_layers %d unsupported", L);
+    LayerGeom g[MAX_LAYERS];
+    chain_geometry(L, 1, &c0, mlp->c_out, g, nullptr);
+    PRB_REQUIRE(fits_pipe(g, 0, L), "sa_group_mlp_max_l0: the chain does not fit one launch");
+    if (b == 0) return 0;
+    ChainIO io;
+    memset(&io, 0, sizeof(io));
+    io.kind = 2; io.split = 0;
+    io.rows = (long)b * npoint * nsample;
+    io.base.mode_in = IN_SA; io.base.mode_out = OUT_SA_MAX;
+    io.base.sa_l0 = 1; io.base.l0_c = c0; io.base.l0_np = round_up(c0, KC); io.base.l0_w = l0_w; io.base.l0_shift = l0_shift;
+    io.base.n = n; io.base.npoint = npoint; io.base.ns = nsample; io.base.c_feat = c_feat;
+    io.base.log_ns = 0;
+    while ((1 << io.base.log_ns) < nsample) ++io.base.log_ns;
+    io.base.xyz = xyz; io.base.new_xyz = new_xyz; io.base.feats_pm = feats_pm; io.base.idx = idx;
+    io.base.out = out; io.base.out_pm = out_pm; io.base.out_stride_c = out_stride_c; io.base.out_c_off = out_c_off;
+    return run_chain(io, mlp, nullptr, 0, (cudaStream_t)stream);
+}
+
 PRB_API int prb_fp_interp_mlp_ws(int b, int n, int m, int c_known, int c_skip, const float *known_pm, const int *idx,
                                  const float *weight, const float *skip, const prb_mlp_desc *mlp, float *out, float *out_pm,
                                  void *workspace, size_t workspace_bytes, void *stream) {

@@ -39,6 +39,8 @@ class _FusedMLP:
         self.desc = None
         self.tensors = None
         self.c_out = None
+        self.proj = None
+        self.l0 = None
 
     @staticmethod
     def supported(mlp: nn.Sequential):
@@ -58,8 +60,11 @@ class _FusedMLP:
                 return False
         return True
 
-    def get(self, mlp: nn.Sequential, kind: int, split: int, device, project_known: bool = False):
-        """project_known (FP chains, kind 1): layer 0 is split by linearity -- interp(known) @ W0k^T == interp(known @ W0k^T) --
+    def get(self, mlp: nn.Sequential, kind: int, split: int, device, project_known: bool = False, layer0: bool = False):
+        """layer0 (SA chains, kind 0, split = c_feat <= 5): layer 0 is taken out of the tensor-core chain -- the gather warps
+        evaluate relu(W0 . [dxyz, f] + shift0) themselves (`self.l0`: weights (c0, 8) with the BN scale folded, shift0 (c0,))
+        and the returned desc is the chain of layers 1 .. L-1 packed as plain rows (kind 2, c_in = c0).
+        project_known (FP chains, kind 1): layer 0 is split by linearity -- interp(known) @ W0k^T == interp(known @ W0k^T) --
         into a per-KNOWN-point projection (a separate, 4x smaller row GEMM: `self.proj`, linear, no shift) and a main chain
         whose layer 0 reads [interp(projected rows) | skip] through the weight [I | W0s]: the gather moves c_out0 instead of
         c_known floats per neighbour and layer 0 contracts over c_out0 + c_skip instead of c_known + c_skip columns."""
@@ -70,7 +75,7 @@ class _FusedMLP:
             if hasattr(layer, "bn"):
                 bn = layer.bn.bn
                 tensors += [bn.weight, bn.bias, bn.running_mean, bn.running_var]
-        key = (kind, split, str(device), _fold_scale(), project_known) + tuple((id(t), t._version) if t is not None else None for t in tensors)
+        key = (kind, split, str(device), _fold_scale(), project_known, layer0) + tuple((id(t), t._version) if t is not None else None for t in tensors)
         if key == self.key:
             return self.desc
         L = len(layers)
@@ -99,6 +104,16 @@ class _FusedMLP:
                 shifts.append(F.pad(sh, (0, pad)))
         lib = C.lib()
         self.proj = None
+        self.l0 = None
+        if layer0:
+            assert _fold_scale() and L >= 2 and kind == 0 and c_in == 3 + split <= L0_IN
+            w0, sh0 = split_layer0(ws[0], shifts[0][:c_out[0]])
+            self.l0 = dict(w=w0.to(device), shift=sh0.to(device), c0=c_out[0])
+            ws, scales, shifts = ws[1:], scales[1:], shifts[1:]
+            kind, split, c_in, L = 2, 0, c_out[0], L - 1
+            c_out_chain = c_out[1:]
+        else:
+            c_out_chain = c_out
         if project_known:
             # ws[0] is (c_out0, c_known + c_skip) with the BN scale already folded in: W0k -> projection, W0s stays
             W0 = ws[0]
@@ -106,7 +121,7 @@ class _FusedMLP:
             self.proj = self._pack(lib, 2, 0, c_known, [c1], [W0[:, :c_known].contiguous()], torch.zeros(_round_up(c1, 32)), device, flags=1)
             ws[0] = torch.cat([torch.eye(c1), W0[:, c_known:]], dim=1).contiguous()
             c_in, split = c1 + (c_in - c_known), c1
-        co_arr = (ctypes.c_int * 3)(*(c_out + [0] * (3 - L)))
+        co_arr = (ctypes.c_int * 3)(*(c_out_chain + [0] * (3 - L)))
         nbytes = lib.prb_mlp_packed_bytes_ex(kind, split, L, c_in, co_arr)
         host = np.zeros(nbytes // 4, dtype=np.float32)
         wp = (ctypes.c_void_p * L)(*[w.data_ptr() for w in ws])
@@ -117,7 +132,7 @@ class _FusedMLP:
         desc = C.MlpDesc()
         desc.num_layers, desc.c_in = L, c_in
         for i in range(3):
-            desc.c_out[i] = c_out[i] if i < L else 0
+            desc.c_out[i] = c_out_chain[i] if i < L else 0
         desc.packed_w, desc.scale, desc.shift = packed.data_ptr(), (None if _fold_scale() else scale.data_ptr()), shift.data_ptr()
         self.key, self.desc, self.tensors, self.c_out = key, desc, (packed, scale, shift), c_out
         return desc
@@ -139,6 +154,37 @@ class _FusedMLP:
             desc.c_out[i] = c_out[i] if i < L else 0
         desc.packed_w, desc.scale, desc.shift, desc.flags = packed.data_ptr(), None, shift.data_ptr(), flags
         return dict(desc=desc, keep=(packed, shift, ws), c_out=c_out, co_arr=co_arr)
+
+
+L0_IN = 8   # layer-0 inputs of the direct form: [dx, dy, dz, up to 5 feature channels] (csrc/mlp_dev.cuh)
+
+
+def split_layer0(w0: torch.Tensor, shift0: torch.Tensor):
+    """layer 0 of an SA chain with c_feat <= 5 for the gather warps: w0 (c0, 3 + c_feat) in the module's column order
+    [xyz, feats], BN scale already folded -> ((c0, L0_IN) zero-padded weights, (c0,) shift), float32, contiguous"""
+    c0, c_in = w0.shape
+    assert c_in <= L0_IN and shift0.shape == (c0,)
+    w = torch.zeros((c0, L0_IN), dtype=torch.float32)
+    w[:, :c_in] = w0.float()
+    return w.contiguous(), shift0.float().contiguous()
+
+
+def _layer0_direct(mlp: nn.Sequential, c_feat: int) -> bool:
+    """SA chain whose layer 0 the gather warps evaluate (prb_sa_group_mlp_max_l0): at most 5 feature channels (a layer 0 of
+    <= 8 FMAs per output, every operand already in the gathering lane), BN scale folded, at least one layer left for the
+    tensor core, and layers 1 .. L-1 fit one launch (the entry does not split chains)"""
+    if c_feat > L0_IN - 3 or not _fold_scale():
+        return False
+    c_out = [layer.conv.out_channels for layer in mlp.children()]
+    if len(c_out) < 2:
+        return False
+    np_ = [_round_up(c, 32) for c in c_out[1:]]
+    last = np_[-1]
+    if last > 512 or sum(np_[:-1]) + (2 * min(last, 64) if len(np_) > 1 else 0) > 512:
+        return False
+    o = C.Options()
+    C.lib().prb_get_thread_options(ctypes.byref(o))
+    return o.mlp_pipeline != 0 and o.mlp_gather == 0      # the layer-0 gather exists in the pipelined kernel only
 
 
 def _attach_pm(t, pm):
@@ -268,13 +314,22 @@ class _PointnetSAModuleBase(nn.Module):
         feats_pm = _point_major(features) if features is not None else None
         if self._fused is None or len(self._fused) != len(self.mlps):
             self._fused = [_FusedMLP() for _ in self.mlps]
-        descs = [f.get(mlp, 0, c_feat, dev) for f, mlp in zip(self._fused, self.mlps)]
+        direct = [_layer0_direct(mlp, c_feat) for mlp in self.mlps]
+        descs = [f.get(mlp, 0, c_feat, dev, layer0=d) for f, mlp, d in zip(self._fused, self.mlps, direct)]
         c_total = sum(f.c_out[-1] for f in self._fused)
         out = torch.empty((B, c_total, npoint), dtype=torch.float32, device=dev)
         out_pm = torch.empty((B, npoint, c_total), dtype=torch.float32, device=dev)   # twin for the next gather
         off = 0
         with torch.cuda.device(dev):
             for desc, fused, idx, ns in zip(descs, self._fused, idxs, nss):
+                if fused.l0 is not None:
+                    l0 = fused.l0
+                    with prof.region("sa_mlp", "%dx%d [%d]+%s l0" % (B * npoint, ns, 3 + c_feat, fused.c_out)):
+                        C.check(lib.prb_sa_group_mlp_max_l0(B, N, npoint, ns, c_feat, C.ptr(xyz), C.ptr(centres), C.ptr(feats_pm),
+                                                            C.ptr(idx), l0["c0"], C.ptr(l0["w"]), C.ptr(l0["shift"]), ctypes.byref(desc),
+                                                            C.ptr(out), C.ptr(out_pm), out.size(1), off, C.stream()), "sa_group_mlp_max_l0")
+                    off += fused.c_out[-1]
+                    continue
                 co_arr = (ctypes.c_int * 3)(*(fused.c_out + [0] * (3 - len(fused.c_out))))
                 wsb = lib.prb_sa_workspace_bytes(B, npoint, ns, c_feat, desc.num_layers, co_arr)
                 ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
